@@ -2,6 +2,7 @@
 """bench.py -- the BASELINE.json benchmarks of the B200 wavelet filter bank.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5] [--gather]
+                    [--dump-outputs DIR]
 
 One "step" = one multi-level forward transform of one batch of synthetic data (per GPU).  Prints ONE JSON line (rank 0).
 
@@ -79,6 +80,44 @@ def make_inverse(mod, cfg):
         return lambda c: mod.waverec3(c, cfg["wavelet"])
     op = mod.MatrixWaverec(cfg["wavelet"])
     return lambda c: op(c)
+
+
+def named_outputs(coeffs) -> dict:
+    """{name: tensor} of a coefficient list [approx, coarsest detail, ..., level-1 detail] as a caller receives it."""
+    top = len(coeffs) - 1
+    out = {"approx": coeffs[0]}
+    for i, el in enumerate(coeffs[1:]):
+        lev = f"detail_level{top - i}"
+        if isinstance(el, torch.Tensor):
+            out[lev] = el
+        elif isinstance(el, dict):
+            out.update((f"{lev}_{k}", el[k]) for k in sorted(el))
+        else:
+            out.update((f"{lev}_{k}", t) for k, t in zip(el._fields, el))
+    return out
+
+
+#: bound on what --dump-outputs writes (bytes of array data)
+DUMP_BYTES = 60 * 10**6
+
+
+def dump_outputs(coeffs, directory: str) -> None:
+    """Write every returned array as <directory>/<name>.npy (its own float dtype).  When all of them together exceed
+    DUMP_BYTES, each one is cut to a fixed sample of its elements -- the same positions for the same shapes in every
+    run (seed 0), flattened in index order -- taking the same share of every array."""
+    import numpy as np
+
+    named = named_outputs(coeffs)
+    total = sum(t.numel() * t.element_size() for t in named.values())
+    share = min(1.0, DUMP_BYTES / total)
+    os.makedirs(directory, exist_ok=True)
+    for name, t in named.items():
+        if share < 1.0:
+            g = torch.Generator().manual_seed(0)
+            k = max(int(t.numel() * share), 1)
+            flat_idx = torch.randint(t.numel(), (k,), generator=g).unique().to(t.device)
+            t = t[torch.unravel_index(flat_idx, t.shape)]
+        np.save(os.path.join(directory, f"{name}.npy"), t.detach().cpu().numpy())
 
 
 def nbytes(ts) -> int:
@@ -180,14 +219,14 @@ def measured_peak_gbs() -> tuple[float, str]:
 # the reference on the host cores
 # --------------------------------------------------------------------------------------------------------------
 def reference_module():
-    """(module, kind): the UNMODIFIED reference from baseline/_ref when it was placed there (baseline/make_ref.py),
+    """(module, kind): the UNMODIFIED reference from oracle/_ref when it was installed there (oracle/make_ref.py),
     else the oracle port (the reference's own torch-CPU operator sequence, pinned bit-identical to it)."""
     try:
-        from baseline.make_ref import import_ref
+        from oracle.make_ref import import_ref
 
         mod = import_ref()
         if mod is not None:
-            return mod, "reference", "unmodified reference (baseline/_ref/ptwt, pywt shim for the filter taps)"
+            return mod, "reference", "unmodified reference (oracle/_ref/ptwt, pywt shim for the filter taps)"
     except Exception:  # noqa: BLE001
         pass
     from oracle import ptwt_port as P
@@ -334,7 +373,11 @@ def main() -> None:
     ap.add_argument("--no-numa", action="store_true")
     ap.add_argument("--no-incumbent", action="store_true", help="skip timing the reference algorithm on the GPU")
     ap.add_argument("--incumbent-batch", type=int, default=16)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the coefficients of the last timed step to DIR/<name>.npy (a fixed sample beyond 60 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = CONFIGS[args.config]
     if args.impl == "reference":
         run_reference(args, cfg)
@@ -441,6 +484,8 @@ def main() -> None:
             worst = max(worst, max(float((a[i:i + 1].cpu() - b).abs().max()) for a, b in zip(fg, want)) / scale)
         parity = {"max_rel_err_vs_oracle": worst, "items_checked": items,
                   "tolerance": 1e-5 if dtype == torch.float32 else 1e-11}
+        if args.dump_outputs:
+            dump_outputs(out, args.dump_outputs)
     del out
 
     _dbg("parity done")

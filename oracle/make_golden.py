@@ -1,10 +1,10 @@
 """Generate tests/golden/*.npz from the UNMODIFIED reference -- TEST INFRASTRUCTURE ONLY.
 
-Runs only in the build container (needs /root/reference); the fixtures are committed so that the
-GPU box, which has no reference, can still check the CUDA path and the oracle port against numbers
+Runs only where the reference is at hand (PTWT_REFERENCE_SRC); the fixtures are committed so that a
+machine without the reference can still check the CUDA path and the oracle port against numbers
 the reference itself produced.
 
-    python -m oracle.make_golden
+    PTWT_REFERENCE_SRC=<reference checkout>/src python -m oracle.make_golden
 """
 from __future__ import annotations
 

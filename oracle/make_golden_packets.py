@@ -1,7 +1,7 @@
 """Generate tests/golden/packet_vectors.* from the UNMODIFIED reference's WaveletPacket / WaveletPacket2D --
-TEST INFRASTRUCTURE ONLY (build container only, needs /root/reference).
+TEST INFRASTRUCTURE ONLY (needs the reference, named by PTWT_REFERENCE_SRC).
 
-    python -m oracle.make_golden_packets
+    PTWT_REFERENCE_SRC=<reference checkout>/src python -m oracle.make_golden_packets
 """
 from __future__ import annotations
 

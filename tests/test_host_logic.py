@@ -4,6 +4,9 @@ Mirrors the error cases of the reference's tests (tests/test_convolution_fwt.py:
 tests/test_convolution_fwt_3.py:167-178; tests/test_matrix_fwt.py:242-245)."""
 from __future__ import annotations
 
+import json
+import sys
+
 import numpy as np
 import pytest
 import torch
@@ -12,8 +15,28 @@ import pytorch_wavelet_toolbox_b200 as wt
 from pytorch_wavelet_toolbox_b200 import _native, _shape
 from pytorch_wavelet_toolbox_b200 import fwt as F
 from pytorch_wavelet_toolbox_b200.matrix_fwt import _level_blocks, _analysis_taps, _level_sizes
+from conftest import GOLDEN
 
 no_gpu = not torch.cuda.is_available()
+
+
+def reference_api() -> dict:
+    return json.loads((GOLDEN / "reference_api.json").read_text())
+
+
+def stand_in_ptwt(monkeypatch):
+    """A ``ptwt`` with the reference's module layout (names bound by value in ``ptwt.packets``), computing with the
+    oracle port -- the reference's own operator sequence -- for install() to find in sys.modules."""
+    import types
+
+    from oracle import ptwt_port as P
+
+    ptwt = types.ModuleType("ptwt")
+    ptwt.packets = types.ModuleType("ptwt.packets")
+    ptwt.wavedec = ptwt.packets.wavedec = P.wavedec
+    monkeypatch.setitem(sys.modules, "ptwt", ptwt)
+    monkeypatch.setitem(sys.modules, "ptwt.packets", ptwt.packets)
+    return ptwt
 
 
 def test_public_surface_and_signatures():
@@ -229,7 +252,7 @@ def test_separable_matrix_nd_argument_errors():
 def test_separable_matrix_level_walk_matches_the_reference_warning(capsys):
     """The level walk of MatrixWavedec2/3 (operator sizes, padded axes, early stop with the reference's
     stderr warning, matmul_transform_2.py:381-405 / matmul_transform_3.py:163-196) is host logic: check it
-    here, and against the unmodified reference when it is importable."""
+    here, and against the warnings the unmodified reference printed (tests/golden/reference_api.json)."""
     from pytorch_wavelet_toolbox_b200.matrix_fwt_nd import _level_sizes
 
     sizes, pads = _level_sizes((33, 20), 4, 2, 2)
@@ -240,54 +263,31 @@ def test_separable_matrix_level_walk_matches_the_reference_warning(capsys):
     ours = capsys.readouterr().err
     assert "only computed up to the decomposition level 2" in ours and "(3, 3,4)" in ours
 
-    from oracle.ref_import import import_reference, reference_available
-    if not reference_available():
-        return
-    ptwt = import_reference()
-    x = torch.randn(12, 9, 16, dtype=torch.float64)
-    ptwt.MatrixWavedec3("db2", 3)(x)
-    ref = capsys.readouterr().err
-    assert ref == ours
+    ref = reference_api()["level_walk_stderr"]          # MatrixWavedec3("db2", 3) on (12, 9, 16), MatrixWavedec2("db3", 3)
+    assert ref[0] == ours                               # on (20, 12)
     _level_sizes((20, 12), 6, 3, 2)
-    ours2 = capsys.readouterr().err
-    ptwt.MatrixWavedec2("db3", 3)(torch.randn(20, 12, dtype=torch.float64))
-    assert capsys.readouterr().err == ours2
+    assert capsys.readouterr().err == ref[1]
 
 
 def test_signatures_equal_the_reference_functions():
     """Every public callable has the parameter names, kinds and defaults of the reference function of the same name
-    (checked against the unmodified reference itself whenever it is importable here)."""
-    import inspect
+    (as the unmodified reference declared them, tests/golden/reference_api.json)."""
+    from oracle.make_golden_api import PACKET_CLASSES, SIGNATURE_CLASSES, SIGNATURE_FUNCTIONS, params
 
-    from oracle.ref_import import import_reference, reference_available
-    if not reference_available():
-        pytest.skip("/root/reference is not present on this machine")
-    ptwt = import_reference()
-
-    def params(fn):
-        return [(n, p.kind, p.default) for n, p in inspect.signature(fn).parameters.items() if n != "self"]
-
-    for name in ("wavedec", "waverec", "wavedec2", "waverec2", "wavedec3", "waverec3", "fswavedec2", "fswavedec3",
-                 "fswaverec2", "fswaverec3"):
-        assert params(getattr(wt, name)) == params(getattr(ptwt, name)), name
-    for name in ("MatrixWavedec", "MatrixWaverec", "MatrixWavedec2", "MatrixWaverec2", "MatrixWavedec3", "MatrixWaverec3"):
-        ours = [q for q in params(getattr(wt, name).__init__) if q[1] is not inspect.Parameter.VAR_KEYWORD]
-        ref = [q for q in params(inspect.unwrap(getattr(ptwt, name).__init__)) if q[1] is not inspect.Parameter.VAR_KEYWORD]
-        assert ours == ref, name
-    for name in ("WaveletPacket", "WaveletPacket2D"):
-        ours = [q[0] for q in params(getattr(wt, name).__init__) if q[1] is not inspect.Parameter.VAR_KEYWORD]
-        ref = [q[0] for q in params(inspect.unwrap(getattr(ptwt, name).__init__))]
-        assert ours == ref, name
+    ref = reference_api()["signatures"]
+    for name in SIGNATURE_FUNCTIONS:
+        assert params(getattr(wt, name)) == ref[name], name
+    for name in SIGNATURE_CLASSES:
+        assert params(getattr(wt, name).__init__) == ref[name], name
+    for name in PACKET_CLASSES:
+        assert [q[0] for q in params(getattr(wt, name).__init__)] == ref[name], name
 
 
-def test_install_leaves_a_cpu_only_machine_alone():
+def test_install_leaves_a_cpu_only_machine_alone(monkeypatch):
     """Without a CUDA device install() must not turn a working CPU ptwt into a failing one (ADVICE round 1)."""
     if torch.cuda.is_available():
         pytest.skip("CUDA device present")
-    from oracle.ref_import import import_reference, reference_available
-    if not reference_available():
-        pytest.skip("/root/reference is not present on this machine")
-    ptwt = import_reference()
+    ptwt = stand_in_ptwt(monkeypatch)
     before = ptwt.wavedec
     with pytest.warns(RuntimeWarning):
         assert wt.install() == []

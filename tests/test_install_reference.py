@@ -1,7 +1,10 @@
-"""install() / uninstall() against the REAL reference package (baseline/_ref, placed by baseline/make_ref.py in the build
-container; it travels to the GPU box with the snapshot): rebinding in ptwt and in the modules that captured the names by
-value, the reference's own packet classes and learnable filters running on the new kernels."""
+"""install() / uninstall(): rebinding in ptwt and in the modules that captured the names by value, against a stand-in
+with the reference's module layout; the REAL reference package (oracle/_ref, installed by oracle/make_ref.py when the
+reference is at hand) for its own packet classes and learnable filters running on the new kernels."""
 from __future__ import annotations
+
+import sys
+import types
 
 import pytest
 import torch
@@ -13,19 +16,43 @@ pytestmark = pytest.mark.gpu
 
 @pytest.fixture
 def ptwt():
-    from baseline.make_ref import import_ref
+    from oracle.make_ref import import_ref
 
     mod = import_ref()
     if mod is None:
-        pytest.skip("baseline/_ref is not present (python baseline/make_ref.py in the build container)")
+        pytest.skip("the reference package is not installed in oracle/_ref (PTWT_REFERENCE_SRC=... python -m oracle.make_ref)")
     yield mod
     wt.uninstall()
 
 
-def test_install_rebinds_and_uninstall_restores(ptwt):
-    import ptwt.packets as packets
-    import ptwt.separable_conv_transform as sep
+@pytest.fixture
+def stand_in_ptwt(monkeypatch):
+    """``ptwt`` with the reference's layout: the names defined in conv_transform(_2) / matmul_transform, re-exported by
+    the package and bound by value in packets (packets.py:34-37) and separable_conv_transform (:33); every function is
+    the oracle port, the reference's own operator sequence."""
+    from oracle import ptwt_port as P
 
+    mods = {name: types.ModuleType(name) for name in ("ptwt", "ptwt.conv_transform", "ptwt.conv_transform_2",
+                                                       "ptwt.matmul_transform", "ptwt.packets",
+                                                       "ptwt.separable_conv_transform")}
+    defined = {"ptwt.conv_transform": ("wavedec", "waverec"), "ptwt.conv_transform_2": ("wavedec2", "waverec2"),
+               "ptwt.matmul_transform": ("MatrixWavedec", "MatrixWaverec")}
+    for modname, names in defined.items():
+        for name in names:
+            setattr(mods[modname], name, getattr(P, name))
+            setattr(mods["ptwt"], name, getattr(P, name))
+    mods["ptwt.packets"].wavedec = mods["ptwt.separable_conv_transform"].wavedec = P.wavedec
+    for modname, mod in mods.items():
+        monkeypatch.setitem(sys.modules, modname, mod)
+        if modname != "ptwt":
+            setattr(mods["ptwt"], modname.split(".")[1], mod)
+    yield mods["ptwt"]
+    wt.uninstall()
+
+
+def test_install_rebinds_and_uninstall_restores(stand_in_ptwt):
+    ptwt = stand_in_ptwt
+    packets, sep = ptwt.packets, ptwt.separable_conv_transform
     ref_wavedec, ref_packets_wavedec, ref_sep_wavedec = ptwt.wavedec, packets.wavedec, sep.wavedec
     replaced = wt.install()
     assert "ptwt.wavedec" in replaced and "ptwt.packets.wavedec" in replaced
@@ -35,7 +62,7 @@ def test_install_rebinds_and_uninstall_restores(ptwt):
     got = ptwt.wavedec2(x, "db2", level=2)                      # the reference's name, our kernels
     wt.uninstall()
     assert ptwt.wavedec is ref_wavedec and packets.wavedec is ref_packets_wavedec and sep.wavedec is ref_sep_wavedec
-    want = ptwt.wavedec2(x.cpu(), "db2", level=2)               # the reference itself on the CPU
+    want = ptwt.wavedec2(x.cpu(), "db2", level=2)               # the reference's operator sequence on the CPU
     flat = lambda c: [c[0]] + [b for lv in c[1:] for b in lv]   # noqa: E731
     scale = max(float(t.abs().max()) for t in flat(want))
     for a, b in zip(flat(got), flat(want)):
